@@ -12,7 +12,7 @@ the fixed-iteration mode (B) of SURVEY.md section 8d - overall_loss_threshold=0,
 iterations and the FLOPs behind the number are known; mode (A), the reference's data-dependent thresholds, is timed
 beside it (`mode_a`) with its per-image iteration counts.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 """
 import argparse
 import json
@@ -328,6 +328,48 @@ def reference_arm(args, config):
     print(json.dumps(line))
 
 
+DUMP_BYTES = 64 << 20          # --dump-outputs budget
+IMAGE_VALUES = 8 << 20         # decoded images up to this many values are written whole (32 MB as float32) ...
+IMAGE_SAMPLE = 2 << 20         # ... larger ones as a sample of this many (value + index: 24 MB)
+SO_IMAGE_SAMPLE = 1 << 20      # the per-box images are always sampled (all of them: 32 x 512 x 512 x 3 values)
+
+
+def seeded_sample(name, a, n_whole, n_sample, out):
+    """out[name] = a as float32 when it has at most n_whole values, else a fixed seeded sample of n_sample values in
+    out[name + "_sample"] with their flat indices in out[name + "_index"]: same arguments, same indices"""
+    import numpy as np
+    flat = np.ascontiguousarray(a).reshape(-1)
+    if flat.size <= n_whole:
+        out[name] = flat.reshape(a.shape).astype(np.float32)
+        return
+    idx = np.sort(np.random.default_rng(0).choice(flat.size, min(n_sample, flat.size), replace=False))
+    out[name + "_sample"] = flat[idx].astype(np.float32)
+    out[name + "_index"] = idx.astype(np.float64)
+
+
+def step_outputs(outs, iters):
+    """what one step's run_batch call handed back, on the host: the final latents [B, 4, h, w], the decoded images
+    [B, H, W, 3] (0..255), the per-box images of phase A (sampled) and the guidance iterations of every image"""
+    import numpy as np
+    d = {"latents": torch.cat([o["latents"] for o in outs], 0).float().cpu().numpy(),
+         "guidance_iterations": np.asarray(iters, dtype=np.float64)}
+    if outs[0].image is not None:
+        seeded_sample("images", np.stack([o.image for o in outs]), IMAGE_VALUES, IMAGE_SAMPLE, d)
+    so = [im for o in outs for im in (o.so_img_list or [])]
+    if so:
+        seeded_sample("so_images", np.stack(so), 0, SO_IMAGE_SAMPLE, d)
+    return d
+
+
+def write_outputs(path, arrays):
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_BYTES, f"--dump-outputs: {total} bytes > {DUMP_BYTES}"
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -346,7 +388,12 @@ def main():
     ap.add_argument("--vae", type=int, default=int(os.environ.get("B200_BENCH_VAE", "1")),
                     help="1: decode every per-box and overall generation with the B200 VAE decoder (synthetic weights) "
                          "inside the timed step, as models/pipelines.py:233,461,591 do")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (final latents, decoded images, a seeded sample of "
+                         "the per-box images, guidance iteration counts) as DIR/<name>.npy, float32/float64, <= 64 MB")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the B200 path computed; --impl reference times a sample of the CPU path")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -415,6 +462,8 @@ def main():
         io["d2h"] = host.numel() * host.element_size()
         if outs[0].image is not None:                     # decoded pictures already crossed to the host in env.decode
             io["d2h"] += sum(o.image.nbytes + sum(im.nbytes for im in (o.so_img_list or [])) for o in outs)
+        if args.dump_outputs:
+            last["outs"] = outs
         st = outs[0]["guidance_state"]
         if wl == "boxdiff":
             last["iters"] = [len(getattr(st, "boxdiff_losses", []))] * len(outs)
@@ -467,6 +516,7 @@ def main():
         log(f"warm-up step {i} done")
     ms, launches, clocks = timed(env_res, args.steps)
     iters_b = list(last["iters"])
+    dump = step_outputs(last.pop("outs"), iters_b) if args.dump_outputs else None
     log(f"timed (resident inputs, fixed 65 iterations): {ms:.1f} ms for {args.steps} step(s)")
     env_host.bytes_out = 0
     k_e2e = min(args.steps, 8)             # bounded: the end-to-end leg repeats the same step with host inputs
@@ -498,6 +548,9 @@ def main():
             line["cpu_baseline"] = cpu_baseline()
             log("cpu baseline done")
         print(json.dumps(line))
+        if dump is not None:
+            write_outputs(args.dump_outputs, dump)
+            log(f"outputs of the last timed step written to {args.dump_outputs}")
     if world > 1:
         dist.destroy_process_group()
 

@@ -16,6 +16,7 @@ The only host<->device traffic inside a step is the per-image loss read-back tha
 (loss.item(), pipelines.py:30).
 """
 import ctypes
+import gc
 import os
 import sys
 import time
@@ -124,8 +125,17 @@ class CudaGraph:
                 rec = owner.__dict__["_graph_pool"] = (torch.cuda.graph_pool_handle(), weakref.WeakSet())
             pool = rec[0]
             rec[1].add(self)
-        with torch.cuda.graph(self.graph, pool=pool):
-            self.out = fn()
+        # no garbage collection while capturing: torch.cuda.graph does not collect before capture_begin, so a collection
+        # triggered inside the capture would run the finalizers of dead objects (graphs and buffers of earlier nets),
+        # and their CUDA calls invalidate the capture
+        gc_was_enabled = gc.isenabled()
+        gc.disable()
+        try:
+            with torch.cuda.graph(self.graph, pool=pool):
+                self.out = fn()
+        finally:
+            if gc_was_enabled:
+                gc.enable()
         CudaGraph.capture_seconds += time.perf_counter() - t0
 
     def __call__(self):

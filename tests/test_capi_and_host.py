@@ -101,28 +101,35 @@ def test_ddim_schedule_matches_oracle():
             assert (mine - b.step(e, t, x)).abs().max() < 2e-5
 
 
-def test_latents_helpers_match_reference():
-    from oracle import ref_loader
-    if not ref_loader.available():
-        pytest.skip("/root/reference not present")
-    r = ref_loader.load()
-    from lgd_b200 import latents as L
+def latents_helper_cases():
+    """(tensor, dx, dy, box) x 50"""
     rng = random.Random(1)
+    g = torch.Generator().manual_seed(1)
     for _ in range(50):
-        t = torch.randn(3, 2, 16, 16)
+        t = torch.randn(3, 2, 16, 16, generator=g)
         dx, dy = rng.uniform(-0.6, 0.6), rng.uniform(-0.6, 0.6)
-        assert torch.equal(L.shift(t, dx, dy), r.utils.shift_tensor(t, dx, dy, offset_normalized=True))
         box = (0.1, 0.2, 0.1 + rng.uniform(0.1, 0.7), 0.2 + rng.uniform(0.1, 0.7))
-        assert torch.equal(L.box_to_mask(box, 64, 64), r.utils.proportion_to_mask(box, 64, 64))
+        yield t, dx, dy, box
+
+
+def test_latents_helpers_match_reference():
+    """utils/utils.py shift_tensor, proportion_to_mask, binary_mask_to_box_mask, binary_mask_to_center, get_centered_box
+    vs latents.py; the reference's outputs are stored in tests/golden/oracle_vs_reference.npz (exact results as
+    digests, see oracle/make_goldens.py vs_reference)"""
+    import test_oracle_vs_reference as T
+    from lgd_b200 import latents as L
+    from lgd_b200.generation.common import centered_box
+    for i, (t, dx, dy, box) in enumerate(latents_helper_cases()):
+        tag = f"latents_{i}"
+        assert T.digest(L.shift(t, dx, dy)) == T.gold(tag + "_shift")
+        assert T.digest(L.box_to_mask(box, 64, 64)) == T.gold(tag + "_box_mask")
         m = L.box_to_mask(box, 16, 16).bool()
-        assert torch.equal(L.mask_to_box_mask(m), r.utils.binary_mask_to_box_mask(m, to_device=False))
+        assert T.digest(L.mask_to_box_mask(m)) == T.gold(tag + "_mask_to_box")
         cx, cy = L.mask_center(m)
-        rx, ry = r.utils.binary_mask_to_center(m, normalize=True)
+        rx, ry = T.gold(tag + "_center")
         assert abs(cx - rx) < 1e-6 and abs(cy - ry) < 1e-6
-        cb = r.utils.get_centered_box(list(box), horizontal_center_only=False, vertical_placement="floor_padding",
-                                      floor_padding=0.2)
-        from lgd_b200.generation.common import centered_box
-        np.testing.assert_allclose(centered_box(box, False, "floor_padding", 0.2), cb, rtol=1e-12)
+        np.testing.assert_allclose(centered_box(box, False, "floor_padding", 0.2), T.gold(tag + "_centered_box"),
+                                   rtol=1e-12)
 
 
 def test_convert_spec_and_synthetic_env():
@@ -164,17 +171,8 @@ def test_fast_schedule_host_logic():
     assert len(s2.timesteps) == 10
 
 
-def test_compose_and_align_match_reference():
-    """utils/latents.py compose_latents (all steps and the fast-schedule prefix) and align_with_bboxes vs latents.py"""
-    import importlib
-    import types
-    from oracle import ref_loader
-    if not ref_loader.available():
-        pytest.skip("/root/reference not present")
-    ref_loader.load()
-    RL = importlib.import_module("utils.latents")
-    RL.torch_device = "cpu"
-    from lgd_b200 import latents as L
+def compose_cases():
+    """(per-box latents [steps + 1, 1, 4, 16, 16] x 3, masks, background latents, steps, boxes)"""
     g = torch.Generator().manual_seed(0)
     steps = 6
     lat = [torch.randn(steps + 1, 1, 4, 16, 16, generator=g) for _ in range(3)]
@@ -184,25 +182,28 @@ def test_compose_and_align_match_reference():
         m[2 + i:9 + i, 1 + 2 * i:8 + 2 * i] = True
         masks.append(m)
     bg = torch.randn(1, 4, 16, 16, generator=g)
-    md = types.SimpleNamespace(unet=None, scheduler=None, dtype=torch.float32)
+    boxes = [(0.05, 0.1, 0.5, 0.6), (0.4, 0.3, 0.9, 0.8), (0.2, 0.5, 0.7, 0.95)]
+    return lat, masks, bg, steps, boxes
+
+
+def test_compose_and_align_match_reference():
+    """utils/latents.py compose_latents (all steps and the fast-schedule prefix) and align_with_bboxes vs latents.py;
+    the reference's outputs are stored in tests/golden/oracle_vs_reference.npz"""
+    import test_oracle_vs_reference as T
+    from lgd_b200 import latents as L
+    lat, masks, bg, steps, boxes = compose_cases()
     for fast in (None, 3):
-        ref_c, ref_fg = RL.compose_latents(md, [x.clone() for x in lat], [m.clone() for m in masks], steps, 1, 128, 128,
-                                           latents_bg=bg.clone(), use_fast_schedule=fast is not None,
-                                           fast_after_steps=fast)
         n = steps if fast is None else fast
         mine_c, mine_fg = L.compose([x[:n + 1] for x in lat], masks, bg, n)
-        assert torch.equal(ref_c, mine_c) and torch.equal(ref_fg, mine_fg)
-    boxes = [(0.05, 0.1, 0.5, 0.6), (0.4, 0.3, 0.9, 0.8), (0.2, 0.5, 0.7, 0.95)]
+        assert T.digest(mine_c) == T.gold(f"compose_fast{fast}_latents")
+        assert T.digest(mine_fg) == T.gold(f"compose_fast{fast}_owner")
     for horizontal_only in (False, True):
-        rl, rm, ro = RL.align_with_bboxes([x.clone() for x in lat], [m.clone() for m in masks], boxes,
-                                          horizontal_shift_only=horizontal_only)
         ml, mm, mo = L.align_to_boxes([x.clone() for x in lat], [m.clone() for m in masks], boxes,
                                       horizontal_only=horizontal_only)
-        for a, b in zip(rl, ml):
-            assert torch.equal(a, b)
-        for a, b in zip(rm, mm):
-            assert torch.equal(a, b)
-        np.testing.assert_allclose(np.array(ro, dtype=np.float64), np.array(mo, dtype=np.float64), rtol=0, atol=1e-7)
+        tag = f"align_h{int(horizontal_only)}"
+        assert [T.digest(a) for a in ml] == T.gold(tag + "_latents").split(",")
+        assert [T.digest(a) for a in mm] == T.gold(tag + "_masks").split(",")
+        np.testing.assert_allclose(np.array(mo, dtype=np.float64), T.gold(tag + "_offsets"), rtol=0, atol=1e-7)
 
 
 def test_boxdiff_tables_and_struct():
@@ -363,3 +364,36 @@ def test_product_path_never_touches_the_oracle():
     arm = [n for n in tree.body if isinstance(n, ast.ClassDef) and n.name == "CpuArm"][0]
     lo, hi = arm.lineno, max(getattr(n, "end_lineno", arm.lineno) for n in ast.walk(arm) if hasattr(n, "end_lineno"))
     assert hits and all(lo <= line <= hi for line, _ in hits), (hits, lo, hi)
+
+
+def test_bench_dump_outputs_host_side(tmp_path):
+    """bench.py --dump-outputs: float32/float64 .npy files within 64 MB, large outputs as the same seeded sample on
+    every call"""
+    import bench
+    from lgd_b200.generation.common import Output
+    rng = np.random.RandomState(0)
+
+    def outs():
+        res = []
+        for b in range(2):
+            o = Output(image=rng.randint(0, 255, size=(64, 64, 3)).astype(np.uint8),
+                       so_img_list=[rng.randint(0, 255, size=(64, 64, 3)).astype(np.uint8) for _ in range(2)])
+            o["latents"] = torch.from_numpy(rng.randn(1, 4, 8, 8).astype(np.float32)).half()
+            res.append(o)
+        return res
+
+    first = outs()
+    a = bench.step_outputs(first, [3, 4])
+    assert a["latents"].shape == (2, 4, 8, 8) and a["images"].shape == (2, 64, 64, 3)
+    assert a["guidance_iterations"].tolist() == [3.0, 4.0]
+    so = np.stack([im for o in first for im in o.so_img_list]).reshape(-1)
+    assert a["so_images_sample"].size == min(so.size, bench.SO_IMAGE_SAMPLE)
+    np.testing.assert_array_equal(a["so_images_sample"], so[a["so_images_index"].astype(np.int64)])
+    b = bench.step_outputs(outs(), [3, 4])
+    np.testing.assert_array_equal(a["so_images_index"], b["so_images_index"])
+    bench.write_outputs(str(tmp_path / "d"), a)
+    for name, v in a.items():
+        got = np.load(tmp_path / "d" / (name + ".npy"))
+        assert got.dtype in (np.float32, np.float64) and np.array_equal(got, v)
+    with pytest.raises(AssertionError):
+        bench.write_outputs(str(tmp_path / "big"), {"x": np.zeros(bench.DUMP_BYTES // 4 + 1, np.float32)})
